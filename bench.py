@@ -1,6 +1,7 @@
 """bench.py — denoising-steps/sec of the Latte hot path (BASELINE.json metric) on N B200s of one node.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dtype fp16|bf16] [--model Latte-XL/2]
+                    [--dump-outputs DIR]
 
 A "step" is one denoising step of `sample/sample.py`: ONE `forward_with_cfg` call on the CFG pair of a
 16x(4x32x32) latent video (B_model = 2) — BASELINE.json configs[1], Latte-XL/2 class-conditional 16x256x256.
@@ -15,6 +16,10 @@ JSON keys beyond the base contract:
   cpu_baseline the oracle port (oracle/latte_oracle.py, torch CPU fp32) timed on this box's host cores, rank 0, N=1
   e2e          same metric through the public module call with HOST pinned buffers: H2D of x, forward, D2H of the result
   --impl reference: times the CPU oracle port only (the reference is pure Python and cannot travel; its restatement can).
+
+--dump-outputs DIR writes what the timed step returned in its last timed call as float32 DIR/<name>.npy (rank 0 only):
+forward_with_cfg.npy for the Latte workload (both impls, same seeded weights and inputs, so the native and reference
+outputs compare directly), t2v_forward.npy for --workload t2v.  Inputs are seeded, so two builds compare output for output.
 """
 from __future__ import annotations
 
@@ -140,44 +145,47 @@ def tune_cpu_threads(O, model_name) -> int:
     return best
 
 
+def dump_outputs(directory, arrays: dict) -> None:
+    """Write each tensor of `arrays` as float32 `directory/<name>.npy` (bench.py --dump-outputs)."""
+    if not directory:
+        return
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, f"{name}.npy"), a.detach().float().cpu().numpy())
+
+
 WORKLOAD = ("{model} class-conditional 16x256x256 sampling step: forward_with_cfg on B_model=2 (1 video x CFG pair) per GPU; "
             "seeded synthetic weights/latents")
 
 
 def run_reference(args):
     """Reference arm: the reference's own CPU implementation of the step on this box's host cores (rank 0 only): W warm-up
-    and K timed `forward_with_cfg` calls, as the main arm, bounded by a wall-clock budget (said in `sample` if it bites)."""
+    and exactly K timed `forward_with_cfg` calls, as the main arm."""
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
     O, cfg, sd, x, t, y = build_case(args.model, 0)
     cores = tune_cpu_threads(O, args.model)
     step, kind, what = cpu_step_factory(O, args.model, cfg, sd, x, t, y)
-    budget_s = 420.0
     W, K = max(args.warmup, 0), args.steps
-    t_start = time.perf_counter()
     with torch.no_grad():
-        warm_done = 0
         for _ in range(W):
-            if warm_done >= 1 and (time.perf_counter() - t_start) > 0.2 * budget_s:
-                break
             step()
-            warm_done += 1
-        done, t1 = 0, time.perf_counter()
-        while done < K and (done == 0 or (time.perf_counter() - t_start) * (1 + 1.0 / max(done, 1)) < budget_s):
-            step()
-            done += 1
+        t1 = time.perf_counter()
+        for _ in range(K):
+            out = step()
         el = time.perf_counter() - t1
-    v = done / el
-    note = "" if (done == K and warm_done == W) else f" (bounded to {budget_s:.0f}s of wall clock: {warm_done}/{W} warm-up, {done}/{K} timed)"
+    dump_outputs(args.dump_outputs, {"forward_with_cfg": out})
+    v = K / el
     print(json.dumps({
-        "impl": "reference", "metric": METRIC, "value": v, "unit": "steps/s", "n_gpus": args.gpus, "steps": done,
-        "warmup": warm_done, "ms_per_step": 1000 * el / done, "higher_is_better": True, "scaling": "weak",
+        "impl": "reference", "metric": METRIC, "value": v, "unit": "steps/s", "n_gpus": args.gpus, "steps": K,
+        "warmup": W, "ms_per_step": 1000 * el / K, "higher_is_better": True, "scaling": "weak",
         "vs_baseline": None, "dtype": "f32", "data": "synthetic",
         "config": {"workload": WORKLOAD.format(model=args.model)},
         "cpu_baseline": {"value": v, "unit": "steps/s", "cores": cores, "kind": kind,
-                         "sample": f"{done} full forward_with_cfg step(s): {what}; {cores} threads = best of a sweep on "
-                                   f"{os.cpu_count()} host threads over the model's own op shapes{note}"},
+                         "sample": f"{K} full forward_with_cfg step(s): {what}; {cores} threads = best of a sweep on "
+                                   f"{os.cpu_count()} host threads over the model's own op shapes"},
         "e2e": {"value": v, "unit": "steps/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
     }), flush=True)
 
@@ -208,10 +216,11 @@ def run_t2v(args):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(K):
-            net(xd, td, encoder_hidden_states=txd, return_dict=False)
+            out = net(xd, td, encoder_hidden_states=txd, return_dict=False)
         e1.record()
         torch.cuda.synchronize()
         ms = e0.elapsed_time(e1) / K
+        dump_outputs(args.dump_outputs, {"t2v_forward": out[0]})
         _lib.profile_enable(True)
         for _ in range(K):
             net(xd, td, encoder_hidden_states=txd, return_dict=False)
@@ -418,7 +427,11 @@ def main():
     ap.add_argument("--no-video", action="store_true", help="skip the measured 250-step video + VAE decode (profiler runs)")
     ap.add_argument("--workload", default="latte", choices=["latte", "t2v"],
                     help="latte = BASELINE configs[1] (the bench line); t2v = configs[3] denoiser step, a secondary measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the output of the last timed step as float32 DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.workload == "t2v":
         return run_t2v(args)
     if args.impl == "reference":
@@ -472,12 +485,14 @@ def main():
         out_host[k].copy_(o, non_blocking=True)
         out_ready[k].record()
 
+    last = {}
+
     def timed(fn, n):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         barrier()
         e0.record()
         for _ in range(n):
-            fn()
+            last["out"] = fn()
         e1.record()
         barrier()
         return sharding.max_over_ranks(e0.elapsed_time(e1), dev)
@@ -492,6 +507,7 @@ def main():
             step_e2e()
         clocks.mark_begin()
         ms_total = timed(step_resident, K)
+        resident_out = last["out"]
         ms_e2e = timed(step_e2e, K)
         clocks.mark_end()
         clk = clocks.stop() if rank == 0 else None
@@ -509,6 +525,8 @@ def main():
         nl = (C.c_int * 4)()
         _lib.check(lib.b200_profile_collect(ms, nl, 4), "b200_profile_collect")
         _lib.profile_enable(False)
+    if rank == 0:
+        dump_outputs(args.dump_outputs, {"forward_with_cfg": resident_out})
 
     # ---- legs every rank takes part in (they end in a collective): frames/s end to end and the sample_ddp batch
     video_leg, ddp_leg, train_leg = None, None, None

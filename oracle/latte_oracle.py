@@ -172,6 +172,14 @@ def make_inputs(cfg: LatteConfig, batch: int, seed: int = 123):
     return x, t, y
 
 
+def subops_inputs(cfg: LatteConfig, seed: int = 99):
+    """Seeded (xs, c) of the sub-op goldens: 3 sequences of 64 tokens and their conditioning vectors."""
+    g = torch.Generator().manual_seed(seed)
+    xs = torch.randn(3, 64, cfg.hidden_size, generator=g)
+    c = torch.randn(3, cfg.hidden_size, generator=g)
+    return xs, c
+
+
 # ----------------------------------------------------------------------------------------------
 # the forward, op by op
 # ----------------------------------------------------------------------------------------------

@@ -25,6 +25,7 @@ ROOT = os.path.dirname(HERE)
 sys.path.insert(0, ROOT)
 sys.path.insert(0, os.path.join(HERE, "ref_shim"))
 
+from oracle import golden as G  # noqa: E402
 from oracle import t2v_oracle as T  # noqa: E402
 
 REF = "/root/reference/models/latte_t2v.py"
@@ -77,7 +78,7 @@ def gen_forward(ref, tag, cfg_kw, batch, text_len, wseed, iseed, out_dir, valid=
     with torch.no_grad():
         out = m(x, t, encoder_hidden_states=text, encoder_attention_mask=mask, enable_temporal_attentions=temporal,
                 return_dict=False)[0]
-    res = dict(out=out.numpy(), t=t.numpy(), x_sum=np.float64(x.double().sum().item()),
+    res = dict(**G.pack("out", out.numpy()), t=t.numpy(), x_sum=np.float64(x.double().sum().item()),
                text_sum=np.float64(text.double().sum().item()),
                cfg=np.array(repr(cfg_kw)), batch=np.int64(batch), text_len=np.int64(text_len), wseed=np.int64(wseed),
                iseed=np.int64(iseed), temporal=np.int64(int(temporal)))

@@ -11,6 +11,7 @@ import numpy as np
 import pytest
 import torch
 
+from oracle import golden as G
 from oracle import latte_oracle as O
 
 pytestmark = pytest.mark.gpu
@@ -37,7 +38,6 @@ CASES = ["latte_tiny64_2_b2.npz", "latte_tiny72_2_b2.npz", "latte_tiny72_2_extra
 @pytest.mark.parametrize("fname", CASES)
 def test_forward_matches_reference_golden(golden_dir, fname):
     g, cfg, sd, net, (x, t, y) = _build(golden_dir, fname)
-    ref = torch.from_numpy(g["out"])
     half = torch.from_numpy(g["out_cfg_half_eps"])
     dev = torch.device("cuda:0")
     xd, td, yd = x.to(dev), t.to(dev), (y.to(dev) if y is not None else None)
@@ -45,8 +45,9 @@ def test_forward_matches_reference_golden(golden_dir, fname):
         for dt, tol in ((torch.float16, 1e-2), (torch.bfloat16, float(g["ref_bf16_maxabs"]))):
             net.compute_dtype = dt
             out = net(xd, td, y=yd).cpu()
-            assert out.shape == ref.shape and out.dtype == torch.float32
-            err = (out - ref).abs().max().item()
+            assert out.dtype == torch.float32
+            got, ref = G.pair(g, "out", out)
+            err = (got - ref).abs().max().item()
             assert err < tol, f"{fname} {dt}: max-abs {err:.3e} >= {tol:.3e}"
             oc = net.forward_with_cfg(xd, td, y=yd, cfg_scale=7.0).cpu()
             b = out.shape[0]
@@ -57,7 +58,8 @@ def test_forward_matches_reference_golden(golden_dir, fname):
     net.half()
     with torch.no_grad():
         o16 = net(xd, td, y=yd)
-    assert o16.dtype == torch.float16 and (o16.float().cpu() - ref).abs().max().item() < 1.5e-2   # vs the fp32-weight golden: includes the weight rounding
+    got, ref = G.pair(g, "out", o16.float().cpu())
+    assert o16.dtype == torch.float16 and (got - ref).abs().max().item() < 1.5e-2   # vs the fp32-weight golden: includes the weight rounding
     if "xl" not in fname:
         # the north_star bound (1e-2) on the path itself: against the oracle evaluated in fp32 on the SAME fp16-rounded weights
         # (sample.py:72-75's model.half()), so that only the kernels' operand rounding is measured

@@ -8,6 +8,7 @@ import numpy as np
 import pytest
 import torch
 
+from oracle import golden as G
 from oracle import latte_oracle as O
 
 
@@ -39,10 +40,10 @@ def test_forward_matches_reference_golden(golden_dir, fname):
     x, t, y = O.make_inputs(cfg, batch, iseed)
     assert abs(float(x.double().sum()) - float(g["x_sum"])) < 1e-9
     out = O.latte_forward(sd, cfg, x, t, y)
-    ref = torch.from_numpy(g["out"])
-    assert out.shape == ref.shape == (batch, cfg.num_frames, cfg.out_channels, cfg.input_size, cfg.input_size)
+    assert out.shape == (batch, cfg.num_frames, cfg.out_channels, cfg.input_size, cfg.input_size)
+    got, ref = G.pair(g, "out", out)
     # same fp32 math, different op order (fused reshape vs einops): tolerance 2e-4 on O(5) outputs
-    assert (out - ref).abs().max().item() < 2e-4
+    assert (got - ref).abs().max().item() < 2e-4
     out_cfg = O.latte_forward_with_cfg(sd, cfg, x, t, y, cfg_scale=7.0)
     half = torch.from_numpy(g["out_cfg_half_eps"])
     assert (out_cfg[: batch // 2, :, :4] - half).abs().max().item() < 1e-3
@@ -55,8 +56,8 @@ def test_fp64_oracle_is_closer_than_bf16_reference(golden_dir):
     g, cfg, batch, wseed, iseed = _load(golden_dir, "latte_tiny72_2_b2.npz")
     sd = O.make_weights(cfg, wseed)
     x, t, y = O.make_inputs(cfg, batch, iseed)
-    out64 = O.latte_forward(sd, cfg, x.double(), t, y, dtype=torch.float64).float()
-    dev = (out64 - torch.from_numpy(g["out"])).abs().max().item()
+    got, ref = G.pair(g, "out", O.latte_forward(sd, cfg, x.double(), t, y, dtype=torch.float64).float())
+    dev = (got - ref).abs().max().item()
     assert dev < 2e-4 < float(g["ref_bf16_maxabs"])
 
 
@@ -64,15 +65,22 @@ def test_subops_match_reference(golden_dir):
     g = np.load(os.path.join(golden_dir, "subops_tiny72.npz"))
     cfg = O.make_config("Latte-tiny72/2", input_size=16, num_frames=4)
     sd = O.make_weights(cfg, 7)
-    xs, c, t = (torch.from_numpy(g[k]) for k in ("xs", "c", "t"))
+    xs, c = O.subops_inputs(cfg)
+    assert abs(float(xs.double().sum()) - float(g["xs_sum"])) < 1e-9
+    assert torch.equal(c, torch.from_numpy(g["c"]))
+    t = torch.from_numpy(g["t"])
     tol = 2e-5
+
+    def err(key, got):
+        got, want = G.pair(g, key, got)
+        return (got - want).abs().max()
     assert (O.timestep_embedding(t) - torch.from_numpy(g["t_freq"])).abs().max() < 1e-6
     assert (O.t_embedder(sd, t, torch.float32) - torch.from_numpy(g["t_emb"])).abs().max() < tol
-    assert (O.transformer_block(sd, 0, xs, c, cfg.num_heads) - torch.from_numpy(g["block0"])).abs().max() < 1e-4
-    assert (O.attention_math(sd, "blocks.0.attn.", xs, cfg.num_heads) - torch.from_numpy(g["attn0"])).abs().max() < tol
-    assert (O.mlp(sd, "blocks.0.mlp.", xs) - torch.from_numpy(g["mlp0"])).abs().max() < tol
+    assert err("block0", O.transformer_block(sd, 0, xs, c, cfg.num_heads)) < 1e-4
+    assert err("attn0", O.attention_math(sd, "blocks.0.attn.", xs, cfg.num_heads)) < tol
+    assert err("mlp0", O.mlp(sd, "blocks.0.mlp.", xs)) < tol
     assert (O.final_layer(sd, xs, c) - torch.from_numpy(g["final"])).abs().max() < 1e-4
-    assert (O.modulate(O.layer_norm(xs), c, c * 0.5) - torch.from_numpy(g["modulate"])).abs().max() < tol
+    assert err("modulate", O.modulate(O.layer_norm(xs), c, c * 0.5)) < tol
     un = O.unpatchify(cfg, torch.arange(2 * 64 * 32, dtype=torch.float32).reshape(2, 64, 32))
     assert torch.equal(un, torch.from_numpy(g["unpatchify"]))
     # sin-cos tables: bit-exact against a freshly initialised reference model

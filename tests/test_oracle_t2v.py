@@ -11,6 +11,7 @@ import numpy as np
 import pytest
 import torch
 
+from oracle import golden as G
 from oracle import t2v_oracle as T
 
 
@@ -42,17 +43,19 @@ CASES = ["tiny_b2_l20", "tiny_b2_l20_notemporal", "tiny_b2_l20_masked", "hd72_b2
 def test_forward_matches_reference_golden(golden_dir, tag):
     g, cfg, sd, x, t, text, mask = load_case(golden_dir, tag)
     out = T.t2v_forward(sd, cfg, x, t, text, enable_temporal=bool(int(g["temporal"])), text_mask=mask)
-    ref = torch.from_numpy(g["out"])
-    assert out.shape == ref.shape
+    out, ref = G.pair(g, "out", out)
     assert (out - ref).abs().max().item() < 5e-4
 
 
 def test_mask_changes_the_output(golden_dir):
     """the masked goldens are not the unmasked ones (the reference really applied the bias)"""
-    a = np.load(os.path.join(golden_dir, "t2v_hd72_b2_l120.npz"))["out"]
-    b = np.load(os.path.join(golden_dir, "t2v_hd72_b2_l120_masked.npz"))["out"]
-    assert np.abs(a[0] - b[0]).max() > 1e-2          # sample 0 keeps 12 of 120 tokens
-    assert np.abs(a[1] - b[1]).max() < 1e-5          # sample 1 keeps all of them
+    shape, idx, a = G.stored(np.load(os.path.join(golden_dir, "t2v_hd72_b2_l120.npz")), "out")
+    shape_m, idx_m, b = G.stored(np.load(os.path.join(golden_dir, "t2v_hd72_b2_l120_masked.npz")), "out")
+    assert shape == shape_m and shape[0] == 2 and np.array_equal(idx, idx_m)
+    d = np.abs(a - b)
+    first = idx < np.prod(shape[1:])      # stored elements of sample 0
+    assert d[first].max() > 1e-2          # sample 0 keeps 12 of 120 tokens
+    assert d[~first].max() < 1e-5         # sample 1 keeps all of them
 
 
 def test_subops_match_reference_classes(golden_dir):

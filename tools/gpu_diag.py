@@ -166,8 +166,9 @@ def _model_case(fname, dtype, also_cfg=True):
     with torch.no_grad():
         out = net(x.to(dev), t.to(dev), y=y.to(dev) if extras == 2 else None)
         torch.cuda.synchronize()
-        ref = torch.from_numpy(gd["out"]).to(dev)
-        stat(f"model {name} {str(dtype)[6:]} vs reference golden (ref's own bf16 dev {float(gd['ref_bf16_maxabs']):.2e})", out, ref, 1e-2)
+        from oracle import golden as G
+        got, ref = G.pair(gd, "out", out)
+        stat(f"model {name} {str(dtype)[6:]} vs reference golden (ref's own bf16 dev {float(gd['ref_bf16_maxabs']):.2e})", got, ref.to(dev), 1e-2)
         if also_cfg:
             oc = net.forward_with_cfg(x.to(dev), t.to(dev), y=y.to(dev) if extras == 2 else None, cfg_scale=7.0)
             stat(f"model {name} {str(dtype)[6:]} forward_with_cfg half eps", oc[: batch // 2, :, :4], torch.from_numpy(gd["out_cfg_half_eps"]).to(dev), 6e-2)
