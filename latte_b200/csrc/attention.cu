@@ -460,8 +460,9 @@ __host__ __device__ inline V3Plan make_v3_plan(int LK, bool tail) {
   return s;
 }
 
-// 2^x for x <= 0 on the FMA pipe: x = n + f, n = round(x), f in [-0.5, 0.5]; 2^f by a degree-4 minimax polynomial
-// (max relative error 2.8e-6), 2^n by adding n to the exponent field.
+// 2^x for x <= 127 on the FMA pipe (arguments below -125 give 2^-125): x = n + f, n = round(x), f in [-0.5, 0.5]; 2^f by
+// a degree-4 minimax polynomial (max relative error 2.8e-6), 2^n by adding n to the exponent field.  The spatial v3 tiles
+// pass x <= 0; the streaming kernel's lazy maximum passes x up to +ST_TAU.
 __device__ __forceinline__ float ex2_poly(float x) {
   x = fmaxf(x, -125.0f);
   const float t = x + 12582912.0f;              // 1.5 * 2^23: the integer n sits in the low mantissa bits
